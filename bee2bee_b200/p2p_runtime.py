@@ -177,6 +177,7 @@ class P2PNode:
     async def _refresh_local_services(self) -> None:
         """A local service whose engine lost its GPU mesh announces itself unhealthy: peers (and we) sort it last."""
         mine = self.providers.setdefault(self.peer_id, {})
+        changed = []
         for name, svc in list(self.local_services.items()):
             try:
                 meta = svc.get_metadata()
@@ -186,9 +187,13 @@ class P2PNode:
             mine[name] = meta
             if meta.get("healthy", True) != was:
                 logger.warning(f"service '{name}' is now {'healthy' if meta.get('healthy', True) else 'UNHEALTHY (GPU mesh aborted)'}")
-                await self._broadcast(P.service_announce(name, meta))
+                changed.append((name, meta))
         mine["health"] = "good" if all((m or {}).get("healthy", True) for k, m in mine.items()
                                        if not k.startswith("_") and isinstance(m, dict)) else "degraded"
+        # our own view is settled before peers hear of the change: a peer that acts on the announce must not find this
+        # node still preferring the service it just declared unhealthy
+        for name, meta in changed:
+            await self._broadcast(P.service_announce(name, meta))
 
     async def _run_health_checks(self) -> None:
         await self._refresh_local_services()

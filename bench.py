@@ -8,6 +8,7 @@ random-init weights, synthetic 16-token prompts) split into N pieces on N B200s.
     python bench.py --impl reference ...     # A: the unmodified reference (baseline/_ref), HFService path
     python bench.py --impl nccl ...          # B: OUR CONSTRUCTED NCCL(+cuBLAS) pipeline (baseline/nccl_pipeline.py)
     python bench.py --config 2|3|4|5 ...     # the other BASELINE.json configs (see CONFIGS below)
+    python bench.py --dump-outputs DIR ...   # also save the last timed step's tokens + logits (.npy): compare two builds
 
 ours (C): every GPU hosts one contiguous layer range ("piece"); N micro-batch groups of
 `--batch` sequences travel through the pieces as a wavefront; the hop between pieces is the
@@ -57,7 +58,14 @@ def parse_args():
     ap.add_argument("--dtype", default=None, choices=["bf16", "fp8", "mxfp8"],
                     help="fp8 = W8A8 e4m3 GEMMs with per-row/per-token scales; mxfp8 = block-scaled (UE8M0 per 32 K) "
                          "tcgen05 kind::mxf8f6f4 GEMMs (secondary configs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, save what the last timed decode step computed as DIR/<name>.npy: "
+                         "tokens.npy (the id sampled for every sequence, float64) and logits.npy (the sampler's input "
+                         "for the sequences of the last micro-batch group, float32; a fixed seeded sample of vocabulary "
+                         "columns, listed in logits_columns.npy, when the whole would exceed 64 MB)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs is only supported with --impl ours")
     cfg = CONFIGS[a.config]
     dflt = dict(model="llama-3-8b", dtype="bf16", batch=32, groups=0, prompt_len=16, steps=64, warmup=8)
     for k, v in dflt.items():
@@ -139,6 +147,28 @@ def measured_peaks():
 
 def synthetic_prompts(n, length, vocab):
     return [[(7 + 131 * i + 31 * j) % (vocab - 300) + 256 for j in range(length)] for i in range(n)]
+
+
+DUMP_BYTES = 64 * 10 ** 6 - 4096        # --dump-outputs budget, with room for the .npy headers
+
+
+def dump_outputs(out_dir, n_seqs, tokens=None, logits=None):
+    """Write the last timed step's sampled ids of the ``n_seqs`` sequences (float64: exact for any vocabulary) and
+    logits (float32) as .npy files.  Logits beyond the budget are cut to a seeded sample of vocabulary columns that is
+    the same in every run of the same shape, so dumps of two builds compare element for element."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    if tokens is not None:
+        np.save(os.path.join(out_dir, "tokens.npy"), np.asarray(tokens, dtype=np.float64))
+    if logits is not None:
+        rows, vocab = logits.shape
+        keep = (DUMP_BYTES - n_seqs * 8) // (rows * 4 + 8)       # the tokens file + an 8-byte index per kept column
+        if keep < vocab:
+            cols = np.sort(np.random.default_rng(0).choice(vocab, size=keep, replace=False))
+            np.save(os.path.join(out_dir, "logits_columns.npy"), cols.astype(np.float64))
+            logits = logits[:, cols]
+        np.save(os.path.join(out_dir, "logits.npy"), np.ascontiguousarray(logits, dtype=np.float32))
 
 
 def gather_objects(obj, world):
@@ -231,6 +261,10 @@ def run_ours(args):
     if rank == 0:
         assert int((win >= 0).all()) and int((win < cfg.vocab_size).all()), "sampler produced out-of-range ids"
         uniq = len(set(win[:, -1].tolist()))
+    if args.dump_outputs and (rank == 0 or runner.last):
+        # the last step's logits buffer holds the last group's rows; nothing has overwritten it since the timed window
+        dump_outputs(args.dump_outputs, total, tokens=win[:, -1].numpy() if rank == 0 else None,
+                     logits=runner.piece.logits[:B, :cfg.vocab_size].cpu().numpy() if runner.last else None)
     runner.release(list(range(total)))
     tok_s = total * K / (ms / 1e3)
     # streamed bytes of ONE group step on this rank: every weight that a decode step reads (the embedding table is
