@@ -342,7 +342,7 @@ class GpuRunner:
                                     v["kv_len"].data_ptr(), sb)
 
         st["body"] = body
-        if self.use_graphs and os.environ.get("B2B_PREFILL_GRAPH", "1") == "1":
+        if self.use_graphs:
             with torch.cuda.stream(self.stream):
                 if self.world == 1:
                     # dry run (allocations, descriptor cache): every row inactive -> no KV / state / token is written

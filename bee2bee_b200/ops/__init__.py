@@ -9,7 +9,6 @@ from __future__ import annotations
 
 import importlib
 import importlib.util
-import os
 from typing import Optional
 
 import torch
@@ -119,10 +118,6 @@ def pick_bn(m_tok: int) -> int:
     return 256 if m_tok > 512 else 128
 
 
-#: 0 restores the round-2 mid-term rule for under-filled prefill GEMMs (128-wide tiles, deep ring, decode split-K heuristic)
-PREFILL_SPLITK = os.environ.get("B2B_PREFILL_SPLITK", "1") == "1"
-
-
 def pick_prefill_tile(n_out: int, m_tok: int, k: int = 0):
     """(token tile, ring depth, cluster split-K) of a prefill GEMM (m_tok > 64), measured on B200 on the Llama-3-8B shapes
     (profiles/prefill_gemm.md).  0 = the tile's default depth / let ``pick_splitk`` decide.
@@ -148,27 +143,14 @@ def pick_prefill_tile(n_out: int, m_tok: int, k: int = 0):
             s *= 2
         return s
 
-    if PREFILL_SPLITK and m_tok >= 256 and k >= 8192 and tiles256 <= NUM_SMS:
+    if m_tok >= 256 and k >= 8192 and tiles256 <= NUM_SMS:
         return 256, 0, split(tiles256, NUM_SMS)
     if tiles128 > NUM_SMS:
         return 128, 3, 1
-    if PREFILL_SPLITK and m_tok >= 256 and k > 0:
+    if m_tok >= 256 and k > 0:
         return 128, 3, split(tiles128, 2 * NUM_SMS)
     return (128 if m_tok <= 512 else 256), 0, 0          # small chunks: not measured, the decode heuristic decides
 
-
-#: cluster size of the TMA-multicast prefill GEMM (2 or 4); correct on hardware but NOT faster (the prefill GEMM is not
-#: L2-bound, profiles/prefill_gemm.md), so default off;
-#: applies to bf16 GEMMs with token tiles of 128 / 256 and no split-K, everything else ignores it
-GEMM_MC = int(os.environ.get("B2B_GEMM_MC", "0"))
-
-#: L2 weight prefetch: built, measured negative and REMOVED from the kernel in round 2 (profiles/l2_prefetch.md; even
-#: switched off its code and parameters cost ~20 us per decode step).  The value is accepted and ignored.
-L2_PREFETCH = 0
-
-#: shared-memory ring depth of the decode GEMMs (0 = per-token-tile default); fewer stages -> more CTAs per SM, so the
-#: next kernel of a PDL chain becomes resident (and prefetches its weights) while the current one still runs
-GEMM_STAGES = int(os.environ.get("B2B_GEMM_STAGES", "0"))
 
 #: tuning hook: {"buf": int64 cuda tensor, "off": 0, "log": []} makes every GEMM record a per-CTA timeline
 TIMELINE = None
@@ -210,7 +192,7 @@ def gemm(w: torch.Tensor, x: torch.Tensor, out: Optional[torch.Tensor] = None, *
          wait_flag: int = 0, wait_epoch: int = 0, signal_flag: int = 0, signal_epoch: int = 0,
          done_counter: int = 0, free_flag: int = 0, bump_epoch: int = 0, ack_flag: int = 0,
          dbg: int = 0, w_scale: Optional[torch.Tensor] = None,
-         sfa: Optional[torch.Tensor] = None, sfb: Optional[torch.Tensor] = None, mc: int = -1, pf: int = -1,
+         sfa: Optional[torch.Tensor] = None, sfb: Optional[torch.Tensor] = None,
          stages: int = -1, free_lag: int = 0, out2_ptr: int = 0,
          fq_out: Optional[torch.Tensor] = None, fq_sf: Optional[torch.Tensor] = None, fq_bn: int = 0,
          sumsq_out: Optional[torch.Tensor] = None, zero_buf: Optional[torch.Tensor] = None,
@@ -233,7 +215,7 @@ def gemm(w: torch.Tensor, x: torch.Tensor, out: Optional[torch.Tensor] = None, *
         else:
             bn = pick_bn(m_tok)
     if stages < 0:
-        stages = GEMM_STAGES if bn <= 64 else 0
+        stages = 0
     if splitk <= 0:
         splitk = pick_splitk(n_out, m_tok, k, bn, epi, stages)
     if epi == EPI_QKV_ROPE or (no_out and fq_out is not None):
@@ -257,8 +239,7 @@ def gemm(w: torch.Tensor, x: torch.Tensor, out: Optional[torch.Tensor] = None, *
     native().gemm(w, x, o_ptr, ldo, epi, bn, splitk, residual_ptr, ld_res, bias, rstd, norm_from_x, eps, act_gelu,
                   out_fp32, q_out, k_cache, v_cache, positions, slots, n_q_heads, n_kv_heads, head_dim, rope_theta,
                   q_scale, wait_flag, wait_epoch, signal_flag, signal_epoch, done_counter, free_flag, bump_epoch,
-                  ack_flag, dbg, w_scale, sfa, sfb, GEMM_MC if mc < 0 else mc,
-                  L2_PREFETCH if pf < 0 else pf, stages, free_lag, out2_ptr,
+                  ack_flag, dbg, w_scale, sfa, sfb, stages, free_lag, out2_ptr,
                   _ptr(fq_out), _ptr(fq_sf), fq_out.shape[1] if fq_out is not None else 0, fq_bn, _ptr(sumsq_out), _ptr(zero_buf),
                   _ptr(sumsq))
     return out

@@ -6,8 +6,8 @@
 // group.  Per KV tile of BKV keys:
 //     S = Q K^T      tcgen05.mma  (A = Q tile, B = K tile, both K-major 128B-swizzled)  -> TMEM, double buffered
 //     P = softmax    4 warps, one TMEM lane (= row) per thread, online max with lazy rescaling
-//     O += P V       tcgen05.mma  (A = P written to swizzled smem as bf16, B = V tile read MN-major:
-//                                  the cache keeps V as [token, d], i.e. N-contiguous)
+//     O += P V       tcgen05.mma  (A = P written back to TMEM as bf16 over the S columns it came from, B = V tile
+//                                  read MN-major: the cache keeps V as [token, d], i.e. N-contiguous)
 // Warp roles: 0 = TMA producer, 1 = TMEM owner + MMA issuer, 2..5 = softmax / correction / epilogue.
 // q is pre-scaled by 1/sqrt(d) and rotated by the QKV GEMM epilogue; K is rotated when appended.
 //
@@ -18,7 +18,6 @@
 #include <cuda.h>
 #include <cuda_fp8.h>
 
-#include <cstdlib>
 #include <type_traits>
 
 #include "common.cuh"
@@ -91,8 +90,8 @@ __device__ __forceinline__ void tmem_st32(uint32_t taddr, const float* v) {
   asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
 }
 
-// EXPERIMENTAL (P_TMEM variant, not yet run on hardware): D[tmem] (+)= A[tmem] * B[smem] -- the A operand (P) is read
-// from tensor memory: lane = row, 16-bit elements packed two per 32-bit column (element 2j in the low half).
+// D[tmem] (+)= A[tmem] * B[smem] -- the A operand (P) is read from tensor memory: lane = row, 16-bit elements packed
+// two per 32-bit column (element 2j in the low half).
 __device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc,
                                              uint32_t accumulate) {
   asm volatile(
@@ -152,33 +151,20 @@ __device__ __forceinline__ void tmem_ld_fence(uint32_t* r) {
                : "memory");
 }
 
-// 2^x on the FMA/ALU pipes (Cody-Waite split + degree-3 minimax polynomial, rel. error 8.8e-5 << bf16 eps).
-// Kept for experiments: moving every other exponential here was SLOWER (660 vs 750 TFLOP/s at T=4096): the
-// softmax warps are issue/latency bound, not MUFU bound (profiles/attention_tc.md).
-__device__ __forceinline__ float exp2_poly(float x) {
-  x = fmaxf(x, -125.f);
-  const float t = __fadd_rd(x, 12582912.f);        // 1.5 * 2^23: floor(x) lands in the low mantissa bits
-  const float f = x - (t - 12582912.f);            // fractional part in [0, 1)
-  float p = fmaf(0.077119089663f, f, 0.227564394474f);
-  p = fmaf(p, f, 0.695146143436f);
-  p = fmaf(p, f, 1.0f);
-  return __uint_as_float(__float_as_uint(p) + (__float_as_uint(t) << 23));
-}
-
 template <int D>
 struct AtcCfg {
   static constexpr int BKV = 64;                                  // keys per tile == one KV page
   static constexpr int kQBytes = 128 * D * 2;
   static constexpr int kKVBytes = BKV * D * 2;
-  static constexpr int kPBytes = 128 * BKV * 2;
+  static constexpr int kPBytes = 128 * BKV * 2;   // P lives in TMEM; the bytes stay: the footprint sets the CTAs per SM
   static constexpr int kSmemBytes = kQBytes + 4 * kKVBytes + kPBytes + 256;
   static constexpr int kTmemCols = (2 * BKV + D <= 256) ? 256 : 512;   // S double buffer + O
   static constexpr int kMinCtas = (D <= 128) ? 2 : 1;                  // two CTAs per SM: one's softmax hides the other's MMAs
 };
 
-// P_TMEM (EXPERIMENTAL, default false): P stays in tensor memory (written over the first BKV/2 columns of the S buffer
-// it was computed from) and feeds the PV MMA as a TMEM A operand; no P tile in shared memory, no fence.proxy.async.
-template <int D, bool SOFTCAP, bool P_TMEM = false>
+// P stays in tensor memory (written over the first BKV/2 columns of the S buffer it was computed from) and feeds the PV
+// MMA as a TMEM A operand.
+template <int D, bool SOFTCAP>
 __global__ void __launch_bounds__(ATC_THREADS, AtcCfg<D>::kMinCtas)
 attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
                        const __grid_constant__ CUtensorMap tm_v, const AttnTcParams p, const int G, const int QB) {
@@ -195,8 +181,7 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_co
   uint8_t* q_s = smem;
   uint8_t* k_s = q_s + Cfg::kQBytes;                       // [2][kKVBytes]
   uint8_t* v_s = k_s + 2 * Cfg::kKVBytes;                  // [2][kKVBytes]
-  uint8_t* p_s = v_s + 2 * Cfg::kKVBytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(p_s + Cfg::kPBytes);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(v_s + 2 * Cfg::kKVBytes + Cfg::kPBytes);
   uint64_t* q_full = bars + 0;
   uint64_t* k_full = bars + 1;     // [2]
   uint64_t* v_full = bars + 3;     // [2]
@@ -319,13 +304,8 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_co
 #pragma unroll
         for (int kk = 0; kk < BKV / 16; ++kk) {
           const uint64_t b = make_sw128_mnmajor_desc(smem_u32(v_s + s * Cfg::kKVBytes + kk * (16 * 128)), BKV * 128);
-          if constexpr (P_TMEM) {
-            // 16 keys of P = 8 packed columns of the S buffer this tile came from
-            umma_bf16_ts(tmem + O_COL, tmem + S_COL + static_cast<uint32_t>(s) * BKV + kk * 8, b, idesc_o, (n > 0 || kk > 0) ? 1u : 0u);
-          } else {
-            const uint64_t a = make_sw128_kmajor_desc(smem_u32(p_s)) + static_cast<uint64_t>(kk * 2);
-            umma_bf16(tmem + O_COL, a, b, idesc_o, (n > 0 || kk > 0) ? 1u : 0u);
-          }
+          // 16 keys of P = 8 packed columns of the S buffer this tile came from
+          umma_bf16_ts(tmem + O_COL, tmem + S_COL + static_cast<uint32_t>(s) * BKV + kk * 8, b, idesc_o, (n > 0 || kk > 0) ? 1u : 0u);
         }
         umma_commit(&v_empty[s]);
         umma_commit(pv_done);
@@ -376,7 +356,7 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_co
         m_ref = mrow;
       }
       if (n > 0) {
-        mbar_wait(pv_done, static_cast<uint32_t>((n - 1) & 1));        // P smem and O are free again
+        mbar_wait(pv_done, static_cast<uint32_t>((n - 1) & 1));        // O is free again
         tc_fence_after();
         if (__any_sync(0xffffffffu, alpha != 1.f)) {
 #pragma unroll 1
@@ -389,39 +369,21 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_co
           }
         }
       }
-      // P = exp2(s - m_ref) -> bf16 -> swizzled K-major smem tile (A operand of the PV MMA)
+      // P = exp2(s - m_ref) -> bf16 pairs -> TMEM (A operand of the PV MMA)
       const float mr = (m_ref == -INFINITY) ? 0.f : m_ref;          // fully masked so far: exp2(-inf - 0) = 0
       float lsum = 0.f;
-      if constexpr (P_TMEM) {
-        uint32_t pk[BKV / 2];            // bf16 pairs: key 2j in the low half of column j
+      uint32_t pk[BKV / 2];              // bf16 pairs: key 2j in the low half of column j
 #pragma unroll
-        for (int j = 0; j < BKV / 2; ++j) {
-          const float p0 = exp2f(__uint_as_float(r[2 * j]) - mr);
-          const float p1 = exp2f(__uint_as_float(r[2 * j + 1]) - mr);
-          lsum += p0 + p1;
-          const __nv_bfloat162 h = __floats2bfloat162_rn(p0, p1);
-          pk[j] = *reinterpret_cast<const uint32_t*>(&h);
-        }
-        static_assert(BKV == 64, "P_TMEM packs one 64-key tile into 32 columns");
-        tmem_st32_bits(s_addr, pk);      // over the (already consumed) scores of this tile
-      } else {
-      uint8_t* ptile = p_s + row * 128;
-#pragma unroll
-      for (int j = 0; j < BKV / 8; ++j) {
-        uint32_t w[4];
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          const float p0 = exp2f(__uint_as_float(r[8 * j + 2 * e]) - mr);
-          const float p1 = exp2f(__uint_as_float(r[8 * j + 2 * e + 1]) - mr);
-          lsum += p0 + p1;
-          const __nv_bfloat162 h = __floats2bfloat162_rn(p0, p1);
-          w[e] = *reinterpret_cast<const uint32_t*>(&h);
-        }
-        *reinterpret_cast<uint4*>(ptile + ((j ^ (row & 7)) * 16)) = make_uint4(w[0], w[1], w[2], w[3]);
+      for (int j = 0; j < BKV / 2; ++j) {
+        const float p0 = exp2f(__uint_as_float(r[2 * j]) - mr);
+        const float p1 = exp2f(__uint_as_float(r[2 * j + 1]) - mr);
+        lsum += p0 + p1;
+        const __nv_bfloat162 h = __floats2bfloat162_rn(p0, p1);
+        pk[j] = *reinterpret_cast<const uint32_t*>(&h);
       }
-      }
+      static_assert(BKV == 64, "one 64-key tile of P packs into 32 TMEM columns");
+      tmem_st32_bits(s_addr, pk);        // over the (already consumed) scores of this tile
       l = l * alpha + lsum;
-      if constexpr (!P_TMEM) fence_proxy_async_smem();   // generic-proxy smem writes -> visible to the tensor core (async proxy)
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(p_ready);
@@ -516,7 +478,7 @@ attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_co
   }
 }
 
-template <int D, bool SOFTCAP, bool P_TMEM>
+template <int D, bool SOFTCAP>
 int launch_tc_cap(const CUtensorMap& tq, const CUtensorMap& tk, const CUtensorMap& tv, const AttnTcParams& p, int G, int QB,
                   int seqs, int qblocks, cudaStream_t s) {
   using Cfg = AtcCfg<D>;
@@ -524,12 +486,12 @@ int launch_tc_cap(const CUtensorMap& tq, const CUtensorMap& tk, const CUtensorMa
   int dev = 0;
   cudaGetDevice(&dev);
   if (dev < 64 && !set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(attn_prefill_tc_kernel<D, SOFTCAP, P_TMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(attn_prefill_tc_kernel<D, SOFTCAP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          Cfg::kSmemBytes);
     if (e != cudaSuccess) return static_cast<int>(e);
     set[dev] = true;
   }
-  return static_cast<int>(launch_kernel(attn_prefill_tc_kernel<D, SOFTCAP, P_TMEM>,
+  return static_cast<int>(launch_kernel(attn_prefill_tc_kernel<D, SOFTCAP>,
                                         dim3(p.splits > 1 ? p.splits : qblocks, p.n_kv, seqs), dim3(ATC_THREADS),
                                         Cfg::kSmemBytes, s, 1, tq, tk, tv, p, G, QB));
 }
@@ -537,14 +499,8 @@ int launch_tc_cap(const CUtensorMap& tq, const CUtensorMap& tk, const CUtensorMa
 template <int D>
 int launch_tc(const CUtensorMap& tq, const CUtensorMap& tk, const CUtensorMap& tv, const AttnTcParams& p, int G, int QB,
               int seqs, int qblocks, cudaStream_t s) {
-  // P in tensor memory (TS-form tcgen05.mma): validated on B200 in round 2 (same error levels, 757 vs 722 TFLOP/s at
-  // T = 4096, profiles/attention_tc.md) -> default on; B2B_ATTN_P_TMEM=0 selects the shared-memory P variant
-  static const bool p_tmem = [] { const char* e = std::getenv("B2B_ATTN_P_TMEM"); return !(e && e[0] == '0'); }();
-  if (p_tmem)
-    return p.softcap > 0.f ? launch_tc_cap<D, true, true>(tq, tk, tv, p, G, QB, seqs, qblocks, s)
-                           : launch_tc_cap<D, false, true>(tq, tk, tv, p, G, QB, seqs, qblocks, s);
-  return p.softcap > 0.f ? launch_tc_cap<D, true, false>(tq, tk, tv, p, G, QB, seqs, qblocks, s)
-                         : launch_tc_cap<D, false, false>(tq, tk, tv, p, G, QB, seqs, qblocks, s);
+  return p.softcap > 0.f ? launch_tc_cap<D, true>(tq, tk, tv, p, G, QB, seqs, qblocks, s)
+                         : launch_tc_cap<D, false>(tq, tk, tv, p, G, QB, seqs, qblocks, s);
 }
 
 }  // namespace

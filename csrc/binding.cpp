@@ -46,7 +46,7 @@ void gemm(const Tensor& w, const Tensor& x, int64_t out_ptr, int64_t ld_out, int
           // handoff
           int64_t wait_flag, int64_t wait_epoch, int64_t signal_flag, int64_t signal_epoch, int64_t done_counter,
           int64_t free_flag, int64_t bump_epoch, int64_t ack_flag, int64_t dbg, const OptT& w_scale,
-          const OptT& sfa, const OptT& sfb, int64_t mc, int64_t pf_tiles, int64_t stages, int64_t free_lag, int64_t out2_ptr,
+          const OptT& sfa, const OptT& sfb, int64_t stages, int64_t free_lag, int64_t out2_ptr,
           // fused MX quantisation of the output / RMSNorm statistics (raw addresses, 0 = off)
           int64_t q_out8, int64_t q_sf, int64_t ld_q, int64_t q_bn, int64_t sumsq_out, int64_t zero_buf, int64_t sumsq) {
   const bool fp8 = w.scalar_type() == at::kFloat8_e4m3fn;
@@ -81,7 +81,6 @@ void gemm(const Tensor& w, const Tensor& x, int64_t out_ptr, int64_t ld_out, int
   p.act_gelu = act_gelu ? 1 : 0;
   p.fp8 = fp8 ? 1 : 0;
   p.stages = static_cast<int8_t>(stages);
-  p.mc = static_cast<int8_t>(mc);      // experimental TMA-multicast cluster (0/1 = off)
   p.w_scale = ptr_or_null<const float>(w_scale);
   p.sfa = fp8 ? ptr_or_null<const uint8_t>(sfa) : nullptr;
   p.sfb = fp8 ? ptr_or_null<const uint8_t>(sfb) : nullptr;

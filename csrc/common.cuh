@@ -35,9 +35,6 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 __device__ __forceinline__ void fence_barrier_init() {
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 }
-__device__ __forceinline__ void fence_proxy_async_smem() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
 __device__ __forceinline__ void fence_proxy_async_all() {
   asm volatile("fence.proxy.async;" ::: "memory");
 }
@@ -90,24 +87,6 @@ __device__ __forceinline__ void tma_load_2d_hint(void* smem_dst, const CUtensorM
       ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0),
       "r"(c1), "l"(policy)
       : "memory");
-}
-// Multicast variant: the box lands at the same shared-memory offset in every CTA of `cta_mask` and completes
-// bytes on the mbarrier at the same offset in each of them.
-__device__ __forceinline__ void tma_load_2d_multicast(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0,
-                                                      int c1, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1),
-      "h"(cta_mask)
-      : "memory");
-}
-// L2-only prefetch of a tile (no shared-memory destination, no mbarrier): keeps HBM busy with the weight tiles a CTA
-// will need beyond its shared-memory ring while the kernel still waits on its producer (PDL / peer flag).
-__device__ __forceinline__ void tma_prefetch_l2_2d(const CUtensorMap* m, int c0, int c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];"
-               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(c0), "r"(c1)
-               : "memory");
 }
 __device__ __forceinline__ uint64_t l2_policy_evict_first() {
   uint64_t p;
@@ -195,15 +174,6 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(
                    smem_u32(bar))
                : "memory");
-}
-// Same, arriving on the mbarrier at this offset in every CTA of `cta_mask` (a stage that is filled by multicast
-// may only be refilled once ALL consumers of the cluster have retired their MMAs on it).
-__device__ __forceinline__ void umma_commit_multicast(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-          smem_u32(bar)),
-      "h"(cta_mask)
-      : "memory");
 }
 // Each thread of the warp reads its own TMEM lane (warp%4 selects the 32-lane
 // quarter via the address), 16 consecutive fp32 columns.

@@ -79,20 +79,13 @@ __device__ __forceinline__ unsigned long long gtime() {
 __device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, 128;" ::: "memory"); }
 
 // QM: 0 = bf16, 1 = fp8 e4m3 with per-row / per-token fp32 scales, 2 = MX fp8 (e4m3 + UE8M0 scale per 32 K)
-// MC: EXPERIMENTAL, untested on hardware in round 1 (default 1 = off).  MC > 1 launches clusters of MC CTAs along the
-//     weight-tile axis; the CTAs share one token tile, each TMA-loads 1/MC of it with `.multicast::cluster` into every
-//     CTA's stage, and a stage is released by all MC consumers (multicast tcgen05.commit).  Cuts the L2 -> SM traffic of the
-//     L2-bound prefill GEMM (profiles/rooflines.md) by up to 2x at MC = 4.
-template <int BN, int EPI, int QM, int MC = 1>
+template <int BN, int EPI, int QM>
 __global__ void __launch_bounds__(192) gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_w,
                                                       const __grid_constant__ CUtensorMap tmap_x,
                                                       const GemmParams p) {
   using Cfg = GemmCfg<BN>;
   constexpr bool FP8 = QM != 0;
   constexpr bool MX = QM == 2;
-  constexpr bool MCAST = MC > 1;
-  constexpr uint16_t MC_MASK = static_cast<uint16_t>((1u << MC) - 1u);
-  static_assert(!MCAST || (QM == 0 && BN % MC == 0 && (BN / MC) % 8 == 0), "multicast: bf16, token tile divisible into 8-row groups");
   const int STAGES = p.stages;            // ring depth (runtime: 2..Cfg::kStages; fewer stages = more CTAs per SM)
   constexpr int STAGE_BYTES = Cfg::kStageBytes;
   constexpr uint32_t TX_BYTES = STAGE_BYTES + (MX ? Cfg::kSfBytes : 0);
@@ -116,7 +109,6 @@ __global__ void __launch_bounds__(192) gemm_tc_kernel(const __grid_constant__ CU
   const int tok0 = blockIdx.y * BN;          // first token of this CTA
   const int splitk = p.splitk;
   const int krank = (splitk > 1) ? static_cast<int>(cluster_ctarank()) : 0;
-  const bool leader = (krank == 0);
   // split-K reduce-scatter: this CTA finishes token columns [col0, col0 + ncol) of the tile (launcher: splitk | BN)
   const int ncol = BN / splitk;
   const int col0 = krank * ncol;
@@ -135,7 +127,7 @@ __global__ void __launch_bounds__(192) gemm_tc_kernel(const __grid_constant__ CU
     if (lane == 0) {
       for (int s = 0; s < STAGES; ++s) {
         mbar_init(&full_bar[s], 1);
-        mbar_init(&empty_bar[s], MCAST ? MC : 1);     // multicast: every consumer of the cluster releases the stage
+        mbar_init(&empty_bar[s], 1);
       }
       mbar_init(tmem_full_bar, 1);
       fence_barrier_init();
@@ -147,14 +139,6 @@ __global__ void __launch_bounds__(192) gemm_tc_kernel(const __grid_constant__ CU
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_s;
-  uint32_t crank = 0;
-  if constexpr (MCAST) {
-    // peers will multicast into this CTA's ring and arrive on its mbarriers: everyone's barriers must be initialised
-    // (and every CTA running) before the first remote operation
-    crank = cluster_ctarank();
-    cluster_arrive_release();
-    cluster_wait_acquire();
-  }
   pdl_launch_dependents();     // the next kernel may start its own set-up / weight prefetch now
   if (threadIdx.x == 0) B2B_DBG(1);
 
@@ -180,10 +164,6 @@ __global__ void __launch_bounds__(192) gemm_tc_kernel(const __grid_constant__ CU
         fence_proxy_async_all();   // peer-written (generic proxy) data -> TMA (async proxy) reads
       }
       for (int i = 0; i < npre; ++i) {
-        if constexpr (MCAST)
-          tma_load_2d_multicast(smem + i * STAGE_BYTES + A_STAGE_BYTES + crank * (BN / MC) * ROW_BYTES, &tmap_x, &full_bar[i],
-                                (kb_begin + i) * BKE, tok0 + static_cast<int>(crank) * (BN / MC), MC_MASK);
-        else
         tma_load_2d_hint(smem + i * STAGE_BYTES + A_STAGE_BYTES, &tmap_x, &full_bar[i], (kb_begin + i) * BKE, tok0,
                          pol_x);
         if constexpr (MX)
@@ -198,10 +178,6 @@ __global__ void __launch_bounds__(192) gemm_tc_kernel(const __grid_constant__ CU
         mbar_arrive_expect_tx(&full_bar[s], TX_BYTES);
         tma_load_2d_hint(smem + s * STAGE_BYTES, &tmap_w, &full_bar[s], (kb_begin + kb) * BKE,
                          tile_n * BM, pol_w);
-        if constexpr (MCAST)
-          tma_load_2d_multicast(smem + s * STAGE_BYTES + A_STAGE_BYTES + crank * (BN / MC) * ROW_BYTES, &tmap_x, &full_bar[s],
-                                (kb_begin + kb) * BKE, tok0 + static_cast<int>(crank) * (BN / MC), MC_MASK);
-        else
         tma_load_2d_hint(smem + s * STAGE_BYTES + A_STAGE_BYTES, &tmap_x, &full_bar[s],
                          (kb_begin + kb) * BKE, tok0, pol_x);
         if constexpr (MX) {
@@ -244,8 +220,7 @@ __global__ void __launch_bounds__(192) gemm_tc_kernel(const __grid_constant__ CU
           else if constexpr (FP8) umma_f8(tmem_base, adesc + 2 * k, bdesc + 2 * k, idesc, (kb > 0 || k > 0) ? 1u : 0u);
           else umma_bf16(tmem_base, adesc + 2 * k, bdesc + 2 * k, idesc, (kb > 0 || k > 0) ? 1u : 0u);
         }
-        if constexpr (MCAST) umma_commit_multicast(&empty_bar[s], MC_MASK);   // every producer of the cluster writes this slot
-        else umma_commit(&empty_bar[s]);               // frees the smem slot when the MMAs retire
+        umma_commit(&empty_bar[s]);                    // frees the smem slot when the MMAs retire
         if (kb == nkb - 1) { umma_commit(tmem_full_bar); B2B_DBG(4); }   // accumulator complete
       }
       __syncwarp();
@@ -609,11 +584,6 @@ __global__ void __launch_bounds__(192) gemm_tc_kernel(const __grid_constant__ CU
     }
   }
 
-  if constexpr (MCAST) {
-    // no CTA may leave while a peer can still multicast into its ring or arrive on its barriers
-    cluster_arrive_release();
-    cluster_wait_acquire();
-  }
   tc_fence_before();
   __syncthreads();
   if (warp == 1) {
@@ -686,34 +656,6 @@ static int launch_bn_epi(const GemmParams& p, const CUtensorMap& tw, const CUten
   }
   return static_cast<int>(launch_kernel(gemm_tc_kernel<BN, EPI, QM>, dim3(p.n_out / BM, (p.m_tok + BN - 1) / BN, p.splitk),
                                         dim3(192), Cfg::smem_bytes(p.stages), stream, static_cast<unsigned>(p.splitk), tw, tx, p));
-}
-
-// EXPERIMENTAL multicast launch (bf16, token tiles of 128 / 256, no split-K): cluster of MC CTAs along grid.x
-template <int BN, int EPI, int MC>
-static int launch_mc(const GemmParams& p, const CUtensorMap& tw, const CUtensorMap& tx_slice, cudaStream_t stream) {
-  using Cfg = GemmCfg<BN>;
-  static bool attr_set[64] = {};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 64 && !attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(gemm_tc_kernel<BN, EPI, 0, MC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         Cfg::kSmemBytes);
-    if (e != cudaSuccess) return static_cast<int>(e);
-    attr_set[dev] = true;
-  }
-  return static_cast<int>(launch_kernel_cx(gemm_tc_kernel<BN, EPI, 0, MC>, dim3(p.n_out / BM, (p.m_tok + BN - 1) / BN, 1),
-                                           dim3(192), Cfg::smem_bytes(p.stages), stream, static_cast<unsigned>(MC), tw, tx_slice, p));
-}
-template <int BN, int MC>
-static int launch_mc_epi(const GemmParams& p, const CUtensorMap& tw, const CUtensorMap& tx_slice, cudaStream_t stream) {
-  switch (p.epi) {
-    case EPI_PLAIN: return launch_mc<BN, EPI_PLAIN, MC>(p, tw, tx_slice, stream);
-    case EPI_RESIDUAL: return launch_mc<BN, EPI_RESIDUAL, MC>(p, tw, tx_slice, stream);
-    case EPI_GLU: return launch_mc<BN, EPI_GLU, MC>(p, tw, tx_slice, stream);
-    case EPI_QKV_ROPE: return launch_mc<BN, EPI_QKV_ROPE, MC>(p, tw, tx_slice, stream);
-    case EPI_GELU: return launch_mc<BN, EPI_GELU, MC>(p, tw, tx_slice, stream);
-    default: return -4;
-  }
 }
 
 // one compact kernel per (token tile, epilogue): a runtime `switch` in the 16x-unrolled epilogue
@@ -828,14 +770,6 @@ int launch_gemm_tc(const GemmParams& p_in, const void* w, const void* x, int bn,
   if (r) return r;
   r = make_tmap(&tx, x, p.m_tok, p.k, p.k, bn, elt);
   if (r) return r;
-  if (p.mc > 1 && !p.fp8 && p.splitk == 1 && (bn == 128 || bn == 256) && (p.mc == 2 || p.mc == 4) &&
-      (p.n_out / BM) % p.mc == 0) {
-    CUtensorMap txs;      // one CTA loads (and multicasts) bn / mc rows of the token tile
-    r = make_tmap(&txs, x, p.m_tok, p.k, p.k, bn / p.mc, elt);
-    if (r) return r;
-    if (bn == 128) return p.mc == 2 ? launch_mc_epi<128, 2>(p, tw, txs, stream) : launch_mc_epi<128, 4>(p, tw, txs, stream);
-    return p.mc == 2 ? launch_mc_epi<256, 2>(p, tw, txs, stream) : launch_mc_epi<256, 4>(p, tw, txs, stream);
-  }
   switch (bn) {
     case 16: return launch_bn<16>(p, tw, tx, stream);
     case 32: return launch_bn<32>(p, tw, tx, stream);

@@ -25,7 +25,6 @@ struct GemmParams {
   int8_t act_gelu;       // EPI_GLU: 0 = SiLU (SwiGLU), 1 = tanh-GELU (GeGLU)
   int8_t fp8;            // operands are e4m3 (W8A8): W [N,K] and X [T,K] one byte per element
   int8_t stages;         // shared-memory ring depth (0 = the token tile's default)
-  int8_t mc;             // EXPERIMENTAL (0/1 = off): cluster of `mc` CTAs along the weight-tile axis shares the token tile by TMA multicast
   const float* w_scale;  // fp8: per-output-row dequant scale [n_out] (activation scale rides in `rstd`)
   // MX fp8 (tcgen05 kind::mxf8f6f4.block_scale): UE8M0 scale per 32 K elements, pre-arranged in 512-byte
   // chunks per (128 rows, 128 K): byte (r % 32) * 16 + (r / 32) * 4 + (k / 32) % 4.  sfa: weights

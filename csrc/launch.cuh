@@ -20,32 +20,6 @@ inline bool pdl_enabled() {
   return g_pdl_mode == 1;
 }
 
-// cluster along x (TMA-multicast GEMM: CTAs that share a token tile)
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_kernel_cx(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                                    unsigned cluster_x, Args... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  int n = 0;
-  attr[n].id = cudaLaunchAttributeClusterDimension;
-  attr[n].val.clusterDim.x = cluster_x;
-  attr[n].val.clusterDim.y = 1;
-  attr[n].val.clusterDim.z = 1;
-  ++n;
-  if (pdl_enabled()) {
-    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n].val.programmaticStreamSerializationAllowed = 1;
-    ++n;
-  }
-  cfg.attrs = attr;
-  cfg.numAttrs = n;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
                                  unsigned cluster_z, Args... args) {

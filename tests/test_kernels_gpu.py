@@ -52,12 +52,13 @@ def test_gemm_splitk_cluster(splitk, m):
     close(ops.gemm(w, x, splitk=splitk), x.float() @ w.float().t())       # cluster / DSMEM kernel
 
 
-@pytest.mark.parametrize("bn,splitk,stages", [(256, 2, 0), (256, 4, 0), (128, 2, 3), (128, 4, 3), (128, 2, 0)])
+@pytest.mark.parametrize("bn,splitk,stages",
+                         [(256, 2, 0), (256, 4, 0), (128, 2, 3), (128, 4, 3), (128, 2, 0), (256, 1, 0), (128, 1, 0)])
 @pytest.mark.parametrize("m", [256, 300, 512])
 def test_gemm_prefill_splitk_tiles(bn, splitk, stages, m):
     """the (token tile, split-K, ring depth) combinations ops.pick_prefill_tile emits for under-filled prefill GEMMs:
-    cluster split-K with the DSMEM reduce-scatter on 128 / 256-wide token tiles, plain and residual epilogues, ragged
-    last token tile"""
+    cluster split-K with the DSMEM reduce-scatter on 128 / 256-wide token tiles, and the same tiles without split-K;
+    plain and residual epilogues, ragged last token tile"""
     w, x, r = bf(512, 4096, scale=0.03), bf(m, 4096), bf(m, 512)
     ref = x.float() @ w.float().t()
     close(ops.gemm(w, x, bn=bn, splitk=splitk, stages=stages), ref)
@@ -510,29 +511,15 @@ def test_dense_layer_forward_backward_on_tensor_cores():
         close(gb, g.mul((zr > 0).float()).sum(0) if act == "relu" else gb, rtol=1e-3, atol=1e-3)
 
 
-# ------------------------------------------------- TMA-multicast cluster GEMM (correct on hardware; not faster, so opt-in)
-@pytest.mark.parametrize("mc", [2, 4])
-@pytest.mark.parametrize("m", [512, 300])
-def test_gemm_multicast_cluster(mc, m):
-    n, k = 1024, 1024
-    w, x, res = bf(n, k, scale=0.05, seed=1), bf(m, k, seed=2), bf(m, n, seed=3)
-    ref = x.float() @ w.float().t()
-    for bn in (128, 256):
-        close(ops.gemm(w, x, bn=bn, splitk=1, mc=mc), ref, rtol=2e-2, atol=2e-2)
-        close(ops.gemm(w, x, bn=bn, splitk=1, mc=mc, epi=ops.EPI_RESIDUAL, residual=res), ref + res.float(), rtol=2e-2, atol=2e-2)
-
-
-@pytest.mark.parametrize("p_tmem", ["1", "0"])
-def test_attention_p_in_tmem_and_smem_variants(p_tmem):
-    """P kept in tensor memory (TS-form tcgen05.mma, the default) and the shared-memory P variant: the numerics
-    script must report the same error levels for both."""
+def test_attention_p_in_tmem():
+    """P kept in tensor memory (TS-form tcgen05.mma): the numerics script must report every case within bf16 error."""
     import re
     import subprocess
     import sys
 
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     out = subprocess.run([sys.executable, os.path.join(root, "tools", "attn_tc_check.py")], capture_output=True, text=True,
-                         timeout=600, env=dict(os.environ, B2B_ATTN_P_TMEM=p_tmem))
+                         timeout=600)
     assert out.returncode == 0, out.stderr[-2000:]
     errs = [float(x) for x in re.findall(r"max_err ([0-9.]+)", out.stdout)]
     assert len(errs) >= 5 and max(errs) < 0.03, out.stdout

@@ -1,6 +1,5 @@
-"""Prefill GEMM throughput (TFLOP/s) on the Llama-3-8B shapes for token counts 512 / 2048 / 4096: token tile 128 / 256,
-plain kernel vs the TMA-multicast cluster variant (MC = 2 / 4 CTAs share one activation tile).  Also a whole-model
-prefill estimate: sum over the four GEMMs x 32 layers."""
+"""Prefill GEMM throughput (TFLOP/s) on the Llama-3-8B shapes for token counts 512 / 4096: token tile 128 / 256 x ring
+depth.  Also a whole-model prefill estimate: sum over the four GEMMs x 32 layers."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -28,17 +27,16 @@ for T in (512, 4096):
         res = torch.randn(T, n, device=dev).bfloat16() if epi == ops.EPI_RESIDUAL else None
         out = torch.empty(T, n // 2 if epi == ops.EPI_GLU else n, device=dev, dtype=torch.bfloat16)
         flops = 2.0 * T * n * k
-        for bn, mc, st in [(128, 0, 0), (128, 0, 3), (128, 0, 2), (256, 0, 0), (256, 0, 3), (256, 0, 2), (256, 2, 0), (256, 2, 2)]:
-            if True:
-                def run(i=0):
-                    ops.gemm(ws[name][i % 3], x, out=out, epi=epi, residual=res, bn=bn, splitk=1, mc=mc, stages=st)
-                try:
-                    us = timed(run)
-                except Exception as e:
-                    print(f"T={T} {name} bn={bn} mc={mc}: FAILED {e}")
-                    continue
-                total.setdefault((bn, mc, st), 0.0)
-                total[(bn, mc, st)] += us
-                print(f"T={T:5d} {name:8s} bn={bn:3d} mc={mc} stages={st}: {us:8.1f} us  {flops / us / 1e6:7.1f} TFLOP/s", flush=True)
+        for bn, st in [(128, 0), (128, 3), (128, 2), (256, 0), (256, 3), (256, 2)]:
+            def run(i=0):
+                ops.gemm(ws[name][i % 3], x, out=out, epi=epi, residual=res, bn=bn, splitk=1, stages=st)
+            try:
+                us = timed(run)
+            except Exception as e:
+                print(f"T={T} {name} bn={bn} stages={st}: FAILED {e}")
+                continue
+            total.setdefault((bn, st), 0.0)
+            total[(bn, st)] += us
+            print(f"T={T:5d} {name:8s} bn={bn:3d} stages={st}: {us:8.1f} us  {flops / us / 1e6:7.1f} TFLOP/s", flush=True)
     for key, us in sorted(total.items()):
-        print(f"T={T:5d} layer GEMMs bn={key[0]} mc={key[1]} stages={key[2]}: {us:8.1f} us -> 32 layers {us * 32 / 1e3:6.2f} ms ({2.0 * T * 7.0e9 / (us * 32) / 1e6:6.1f} TFLOP/s on the 7.0 G layer params)")
+        print(f"T={T:5d} layer GEMMs bn={key[0]} stages={key[1]}: {us:8.1f} us -> 32 layers {us * 32 / 1e3:6.2f} ms ({2.0 * T * 7.0e9 / (us * 32) / 1e6:6.1f} TFLOP/s on the 7.0 G layer params)")
